@@ -17,6 +17,8 @@ A "step" = one pass of the whole RX hot path (carrier sense -> LTS -> OFDM demod
                topologies of SURVEY.md §8(d): one thread, the reference's two-thread pipeline, all cores.
 `--impl reference` times that CPU implementation alone.  Before any timing the result of every unique slot is compared field by field
 (status, rate, length, FCS, symbol count, detect index, CFO estimate, bytes) with the CPU oracle on the same IQ.
+`--dump-outputs DIR` writes what the last timed step computed (rank 0's verdicts and PSDU bytes of a fixed, seeded sample of slots) to
+DIR/<name>.npy; the input is seeded, so two builds run with the same arguments can be compared output for output.
 Multi-GPU (torchrun): slots are independent, so every rank decodes its own F slots (weak scaling, no data-path collective in `value` / `e2e`).
 """
 import argparse, json, os, re, subprocess, sys, time, threading
@@ -24,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 SLOT = 9824            # 9760 samples of PPDU + 64 zero samples of gap (32 before, 32 after)
 PSDU = 1500
@@ -231,6 +234,21 @@ def oracle_gate(eng, torch, iq_u, ps_u, U, res_dev, out_dev, ncores, rank):
     oracle_gate.rerun = int(len(idx))
     return U
 
+DUMP_SLOTS = 4096      # 4096 x (1500 float32 bytes + 9 float64 fields) = 25 MB
+
+def sample_outputs(torch, res_dev, out_dev):
+    """What a caller of the timed path receives — the verdict fields and the PSDU bytes of every slot — for a fixed, seeded sample of
+    DUMP_SLOTS slots (all of them when there are fewer), as float64 / float32 arrays by name."""
+    from sora_b200 import api
+    F = res_dev.shape[0]
+    idx = np.arange(F) if F <= DUMP_SLOTS else np.sort(np.random.default_rng(0xD0).choice(F, DUMP_SLOTS, replace=False))
+    it = torch.from_numpy(idx).to(res_dev.device)
+    res = res_dev.index_select(0, it).cpu().numpy().view(api.RESULT_DTYPE).reshape(-1)
+    arrays = {"slot_index": idx.astype(np.float64), "psdu": out_dev.index_select(0, it).cpu().numpy().astype(np.float32)}
+    for k in api.RESULT_DTYPE.names:
+        arrays["result_" + k] = res[k].astype(np.float64)
+    return arrays
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -254,7 +272,9 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-mgpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (rank 0, a seeded sample of at most %d slots)" % DUMP_SLOTS)
     args = ap.parse_args()
+    if args.steps < 1: ap.error("--steps must be at least 1")
     if args.warmup < 3: args.warmup = 3
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -318,9 +338,13 @@ def main():
     for _ in range(args.steps):
         step_dev()
     e1.record(stream); torch.cuda.synchronize()
-    if dist: dist.barrier()
     ms_total = e0.elapsed_time(e1)
     launches = eng.launches - l0
+    if args.dump_outputs and rank == 0:                    # before the passes below write the output buffers again
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in sample_outputs(torch, res_dev, out_dev).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+    if dist: dist.barrier()
     # per-kernel times of the dominant kernel, measured live with CUDA events on the launch stream (extra pass, same inputs)
     nk = max(3, min(args.steps, 5))
     eng.set_option("chunk_frames", 0); eng.set_option("chunk_frames_device", 0)   # un-pipelined pass: kernels back to back on one stream

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Known-answer vectors of the reference's LEGACY 802.11a transmitter at all eight rates, made from the reference's own lookup tables.
 
-Runs only in the build container (needs /root/reference).  The data-path stages of BB11ATxFrameMod are table driven: scrambler
+The data-path stages of BB11ATxFrameMod are table driven: scrambler
 (lutst/scramble_11a.c), convolutional encoder with puncturing (conv_encoder_{1_2,2_3,3_4}.c), interleaver (interleave_{6,12,24,48}m.c),
 mapper (mapa_{bpsk,qpsk,16qam,64qam}.c), pilot polarity (pilotsgn.c), preamble (preamble40_11a.c).  This script reads those tables as DATA
 and drives them exactly like the reference's C code does (atx_tpl.h Scramble11a, convenc.h ConvEncode_*, ainterleave.h Interleave*, amap.h
@@ -9,21 +9,32 @@ Map*_11a, addpilot.h, ofdmsymbol.h Generate*Symbol incl. the two alternating 9 M
 the oracle is the fixed-point IFFT<128> (oracle `ifft128`, itself pinned by usr/HwVeri/data/ofdm.bin).  Outputs, under tests/golden/legacy_tx/:
   legacy_tx_<kbps>.i8   complex int8 samples (640 + 160 (1 + nsym) + 8) of one frame per rate
   legacy_tx_<kbps>.bin  the frame body (without FCS) that was modulated
+  lutst_tables.npz      the tables it read, as data: the CPU suite regenerates every vector from them without the reference tree
 The CPU suite then requires oracle/tx11a_legacy.cpp (function-driven restatement) to reproduce every file sample for sample, and the receive
 oracle and the GPU to decode every file to its body: table-derived vectors for the rates the reference ships no waveform of (incl. 54 Mbps)."""
 import os, re, sys, zlib, numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__)); ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
-REF = "/root/reference/kernel/bb/dot11a/lutst/"
+TABLES = ("scramble_11a", "conv_encoder_1_2", "conv_encoder_2_3", "conv_encoder_3_4", "interleave_6m", "interleave_12m",
+          "interleave_24m", "interleave_48m", "mapa_bpsk", "mapa_qpsk", "mapa_16qam", "mapa_64qam", "pilotsgn", "preamble40_11a")
+STORED = os.path.join(HERE, "legacy_tx", "lutst_tables.npz")
 
-def table(name):
-    t = open(REF + name).read(); body = t[t.index("{", t.index("=")):]
+def table(ref, name):
+    """One lookup table of kernel/bb/dot11a/lutst/<name>.c under the reference root `ref` (the values of its initialiser)."""
+    t = open(os.path.join(ref, "kernel/bb/dot11a/lutst", name + ".c")).read(); body = t[t.index("{", t.index("=")):]
     return np.array([int(x, 0) for x in re.findall(r"-?(?:0x[0-9a-fA-F]+|\d+)", body)], dtype=np.int64)
 
-def build():
+def stored_tables():
+    with np.load(STORED) as z: return {k: z[k].astype(np.int64) for k in TABLES}
+
+def save_tables(T):
+    """Each table in the narrowest integer type that holds it (stored_tables() widens them back to int64)."""
+    narrow = lambda v: v.astype(next(t for t in (np.int8, np.uint8, np.int16, np.uint16, np.int32, np.uint32) if np.iinfo(t).min <= v.min() and v.max() <= np.iinfo(t).max))
+    np.savez_compressed(STORED, **{k: narrow(T[k]) for k in TABLES})
+
+def build(T):
+    """T: table name -> int64 values (table() per name, or stored_tables()).  Returns frame(body, kbps) -> int8 [n, 2]."""
     import oracle_py
-    T = {k: table(k + ".c") for k in ("scramble_11a", "conv_encoder_1_2", "conv_encoder_2_3", "conv_encoder_3_4", "interleave_6m", "interleave_12m",
-                                      "interleave_24m", "interleave_48m", "mapa_bpsk", "mapa_qpsk", "mapa_16qam", "mapa_64qam", "pilotsgn", "preamble40_11a")}
     SCR = T["scramble_11a"]; PRE = T["preamble40_11a"].reshape(-1, 2)
     MAP = {1: T["mapa_bpsk"].reshape(-1, 8, 2), 2: T["mapa_qpsk"].reshape(-1, 4, 2), 4: T["mapa_16qam"].reshape(-1, 2, 2), 6: T["mapa_64qam"].reshape(-1, 2, 2)}
     IL = {1: (T["interleave_6m"].reshape(-1, 6), 6, 3, 2), 2: (T["interleave_12m"].reshape(-1, 3), 12, 3, 4),
@@ -123,8 +134,11 @@ def build():
     return frame
 
 if __name__ == "__main__":
-    frame = build()
+    # usage: python tests/golden/make_legacy_tx_vectors.py REFERENCE_ROOT
+    T = {k: table(sys.argv[1], k) for k in TABLES}
     d = os.path.join(HERE, "legacy_tx"); os.makedirs(d, exist_ok=True)
+    save_tables(T)
+    frame = build(T)
     rng = np.random.default_rng(0x11A)
     for kbps, n in ((6000, 40), (9000, 57), (12000, 64), (18000, 77), (24000, 100), (36000, 131), (48000, 190), (54000, 211)):
         body = rng.integers(0, 256, n).astype(np.uint8)

@@ -1,27 +1,21 @@
 """CPU tests of the 802.11n 2x2 oracle (no GPU): tables against the reference headers, SIG parsing, loop-back at MCS 8..10."""
-import os, sys, numpy as np, pytest
+import numpy as np, pytest
 import oracle_py
 from sora_b200 import synth
 
-REF = "/root/reference"
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_tables_vs_reference_headers_11n():
-    import refcheck as rc
+    """The oracle's 802.11n tables against the reference headers' (golden/ref_digests.json)."""
+    import golden_vectors as gv
     T = oracle_py.tables11n()
-    d = rc.ref_demap_11n()
-    assert (d["bpsk"] == T["demap"]).all() and (d["qpsk"] == T["demap"]).all()
-    assert (rc.ref_crc8() == T["crc8"]).all()
+    assert gv.ref_table_equals("demap11n_bpsk", T["demap"]) and gv.ref_table_equals("demap11n_qpsk", T["demap"])
+    assert gv.ref_table_equals("LUT_CRC8", T["crc8"])
     for q, name in enumerate(("BPSK", "QPSK")):
         for s in range(2):
-            ref = rc.ref_deinterleave_11n(f"{name}_S{s}")
-            assert (ref == T["deint"][q, s, :len(ref)]).all() and len(ref) == 52 * (q + 1), (name, s)
-            assert (synth.ht_interleave_map(q + 1, s) == ref).all()        # modulator and receiver agree on the permutation
-    lp, hp = rc.ref_ltf_masks()
-    assert (lp == T["lltf_sign"].astype(bool)).all() and (hp == T["htltf_sign"].astype(bool)).all()
-    nd = rc.ref_ht_ndbps()
-    assert {m: nd[m][1] for m in (8, 9, 10)} == {m: synth.HT_MCS[m][2] for m in (8, 9, 10)}
+            assert gv.ref_table_equals(f"deint11n_{name}_S{s}", T["deint"][q, s, :52 * (q + 1)]), (name, s)
+            assert gv.ref_table_equals(f"deint11n_{name}_S{s}", synth.ht_interleave_map(q + 1, s))      # modulator and receiver agree on the permutation
+    assert gv.ref_table_equals("lltf_plus", T["lltf_sign"].astype(bool)) and gv.ref_table_equals("htltf_plus", T["htltf_sign"].astype(bool))
+    assert gv.ref_table_equals("DOT11N_NDBPS_MCS8_14", [synth.HT_MCS[m][2] for m in range(8, 15)])
 
 def test_dsp_math_tables_closed_form():
     T = oracle_py.tables11n()

@@ -4,10 +4,8 @@ behaviour by default and opens the gate with set_ht_mcs_limit(15) (SURVEY.md §8
 restated modulator graph against the restated receive graph, and an independent float clause-20 modulator."""
 import os, sys, zlib, numpy as np, pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tools"))
 import oracle_py
 from sora_b200 import synth
-REF = "/root/reference"
 
 @pytest.fixture()
 def qam_enabled():
@@ -15,20 +13,17 @@ def qam_enabled():
     yield
     oracle_py.set_ht_mcs_limit(11)
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_qam_tables_vs_reference_headers():
-    import refcheck as rc
+    """The oracle's 16-/64-QAM demap and HT deinterleave tables against the reference headers' (golden/ref_digests.json)."""
+    import golden_vectors as gv
     T = oracle_py.tables11n()
-    t = rc._read("kernel/bb/Brick11/src/dsp_demap.h"); t = t[t.index("This LUT is constructed"):]
-    for i, n in enumerate(("16qam1", "16qam2")): assert (np.array(rc.parse_array(t, "dsp_demapper::lookup_table_" + n)) == T["demap16"][i]).all(), n
-    for i, n in enumerate(("64qam1", "64qam2", "64qam3")): assert (np.array(rc.parse_array(t, "dsp_demapper::lookup_table_" + n)) == T["demap64"][i]).all(), n
+    for i, n in enumerate(("16qam1", "16qam2")): assert gv.ref_table_equals("demap11n_" + n, T["demap16"][i]), n
+    for i, n in enumerate(("64qam1", "64qam2", "64qam3")): assert gv.ref_table_equals("demap11n_" + n, T["demap64"][i]), n
     for q, (name, nb) in enumerate((("BPSK", 1), ("QPSK", 2), ("QAM16", 4), ("QAM64", 6))):
         for s in range(2):
-            ref = rc.ref_deinterleave_11n(f"{name}_S{s}")
-            assert len(ref) == 52 * nb and (ref == T["deint"][q, s, :len(ref)]).all(), (name, s)
-            assert (synth.ht_interleave_map(nb, s) == ref).all()            # the independent modulator uses the same permutation
-    nd = rc.ref_ht_ndbps()
-    assert {m: nd[m][1] for m in range(8, 15)} == {m: synth.HT_MCS[m][2] for m in range(8, 15)}
+            assert gv.ref_table_equals(f"deint11n_{name}_S{s}", T["deint"][q, s, :52 * nb]), (name, s)
+            assert gv.ref_table_equals(f"deint11n_{name}_S{s}", synth.ht_interleave_map(nb, s))       # the independent modulator uses the same permutation
+    assert gv.ref_table_equals("DOT11N_NDBPS_MCS8_14", [synth.HT_MCS[m][2] for m in range(8, 15)])
 
 def _rx(o0, o1, chan, noise, seed=1, lead=400, trail=300):
     a = o0[:, 0] + 1j * o0[:, 1]; b = o1[:, 0] + 1j * o1[:, 1]

@@ -5,7 +5,6 @@ import oracle_py
 from sora_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 def _rx(samples8, lead=400, trail=400):
@@ -45,15 +44,14 @@ def test_near_match_with_reference_modulator_output():
     assert np.abs(mine[inner] - gold[inner]).max() <= 1
     assert (mine == gold).all(1).mean() > 0.93
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_tx_tables_vs_reference():
-    import refcheck as rc
+    """The transmit FFT tables against the reference headers' (golden/ref_digests.json)."""
+    import refcheck as rc, golden_vectors as gv
     for N in (128, 32):
         for M in (1, 2, 3):
-            assert (rc.ref_twiddle(N, M)[:N // 4] == rc.gen_twiddle(N, M)).all()
-    assert (rc.ref_bitrev(128) == np.array([int(format(i, "07b")[::-1], 2) for i in range(128)])).all()
-    t8 = np.array(rc.parse_array(rc._read("kernel/core/inc/fft_lut_twiddle.h"), "wFFTLUT8")).reshape(-1, 2)
-    assert (t8 == np.array([[32767, 0], [23169, -23169], [32767, 0], [-23169, -23169]])).all()
+            assert gv.ref_table_equals(f"twiddle_{N}_{M}", rc.gen_twiddle(N, M)), (N, M)
+    assert gv.ref_table_equals("bitrev_128", [int(format(i, "07b")[::-1], 2) for i in range(128)])
+    assert gv.ref_table_equals("twiddle_8", [[32767, 0], [23169, -23169], [32767, 0], [-23169, -23169]])
 
 
 # ---- the reference's LEGACY transmitter (BB11ATxFrameMod): pinned by its own output file and by vectors made from its own tables ------------
@@ -84,16 +82,17 @@ def test_legacy_tx_vectors_from_reference_tables(kbps):
     assert len(res) == 1 and res[0]["status"] == 1 and res[0]["rate_kbps"] == kbps and res[0]["length"] == len(body) + 4
     assert bytes(out[0, :len(body)]) == bytes(body)
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
 def test_legacy_tx_vectors_regenerate_from_the_reference():
+    """The vectors are what the reference's own transmit lookup tables (kept as data in legacy_tx/lutst_tables.npz) make."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("mk", os.path.join(GOLD, "make_legacy_tx_vectors.py")); mk = importlib.util.module_from_spec(spec); spec.loader.exec_module(mk)
-    frame = mk.build()
+    T = mk.stored_tables()
+    frame = mk.build(T)
     for kbps in (9000, 54000):
         body = np.fromfile(os.path.join(GOLD, "legacy_tx", f"legacy_tx_{kbps}.bin"), np.uint8)
         assert (frame(body, kbps) == np.fromfile(os.path.join(GOLD, "legacy_tx", f"legacy_tx_{kbps}.i8"), np.int8).reshape(-1, 2)).all()
     pre = np.fromfile(os.path.join(GOLD, "preamble40_11a.i16"), np.int16)
-    assert (pre == mk.table("preamble40_11a.c")).all()
+    assert (pre == T["preamble40_11a"]).all()
 
 def test_legacy_tx_ack_frame_round_trip():
     """BB11AModulateACK's path (BB11ATxBufferMod6M: the buffer already ends in its FCS): the 14-byte ACK of the Dot11ADummy fixtures."""

@@ -1,10 +1,8 @@
 """CPU tests of the 802.11b transmit restatement (oracle/tx11b.cpp): stage tables rebuilt from the reference's formulas, the
 shaper's impulse response, and the fixed-point TX -> fixed-point RX round trip at all four rates through the receive oracle (which
 is pinned by the reference's own *.mf.bin captures)."""
-import os, sys, zlib, numpy as np, pytest
+import numpy as np, pytest
 import oracle_py
-
-REF = "/root/reference"
 
 def _rx(samples8, lead=300, trail=600):
     iq = np.concatenate([np.zeros((lead, 2), np.int16), samples8.astype(np.int16) << 8, np.zeros((trail, 2), np.int16)])
@@ -64,11 +62,9 @@ def test_plcp_length_extension_bit():
         res, out = _rx(oracle_py.tx11b_modulate(p, 11000))
         assert res["status"] == 1 and res["length"] == L + 4 and (out[:L] == p).all(), (L, res)
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_tx11b_constants_vs_reference():
-    src = open(os.path.join(REF, "kernel/bb/Brick11/src/barkerspread.hpp")).read()
-    assert "{ 1, -1, 1, 1, -1, 1, 1, 1, -1, -1, -1 }" in src
-    cck = open(os.path.join(REF, "kernel/bb/Brick11/src/cck.hpp")).read()
-    assert "DQPSKEncode[] = { {1, 0}, {0, -1}, {0, 1}, {-1, 0} }" in cck and "CCK11D3D2[] = { {1, 0}, {-1, 0}, {0, 1}, {0, -1} }" in cck
-    plcp = open(os.path.join(REF, "kernel/inc/dot11_plcp.h")).read()
-    assert "DOT11B_PLCP_LONG_TX_SCRAMBLER_REGISTER          0x6C" in plcp and "DOT11B_PLCP_LONG_PREAMBLE_SFD                   0xF3A0" in plcp
+    """The constants oracle/tx11b.cpp restates, against the reference's barkerspread.hpp, cck.hpp and dot11_plcp.h (golden/ref_digests.json)."""
+    import golden_vectors as gv
+    assert gv.ref_table_equals("Barker11", [1, -1, 1, 1, -1, 1, 1, 1, -1, -1, -1])
+    assert gv.ref_table_equals("DQPSKEncode", [[1, 0], [0, -1], [0, 1], [-1, 0]]) and gv.ref_table_equals("CCK11D3D2", [[1, 0], [-1, 0], [0, 1], [0, -1]])
+    assert gv.ref_table_equals("DOT11B_PLCP_LONG_TX_SCRAMBLER_REGISTER", [0x6C]) and gv.ref_table_equals("DOT11B_PLCP_LONG_PREAMBLE_SFD", [0xF3A0])

@@ -1,5 +1,5 @@
-"""The legacy 802.11b transmit filter (BB11BPMDSpreadFIR4SSE, kernel/bb/dot11b/bbb_fir.c) — the oracle's restatement against the reference's
-own compiled code (oracle/_ref, built by oracle/build_ref.sh from the reference source where it lies) and against vectors that code made."""
+"""The legacy 802.11b transmit filter (BB11BPMDSpreadFIR4SSE, kernel/bb/dot11b/bbb_fir.c) — the oracle's restatement against what the reference's
+own compiled code (oracle/build_ref.sh) made: vectors under golden/fir37 and digests of its output on seeded inputs (golden/ref_digests.json)."""
 import os, sys, numpy as np, pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import oracle_py
@@ -13,15 +13,10 @@ def test_restatement_reproduces_vectors_made_by_the_reference_code(name):
     assert (oracle_py.fir37_legacy(x, 0) == y).all()
     if name == "saturating": assert y.max() == 127 and y.min() == -128        # the vector does reach both rails
 
-@pytest.mark.skipif(not oracle_py.ref_fir37_available(), reason="oracle/_ref not built (needs the reference tree: oracle/build_ref.sh)")
 def test_restatement_equals_the_compiled_reference_body():
-    rng = np.random.default_rng(5)
-    for n in (0, 8, 16, 24, 64, 1000 // 8 * 8, 40000):
-        for kind in range(3):
-            if kind == 0: x = rng.integers(-128, 128, (n, 2)).astype(np.int8)
-            elif kind == 1: x = np.where(rng.integers(0, 2, (n, 2)) > 0, 127, -128).astype(np.int8)
-            else: x = np.zeros((n, 2), np.int8); x[::4, 0] = np.where(rng.integers(0, 2, (n + 3) // 4) > 0, 127, -128)
-            assert (oracle_py.fir37_legacy(x, 0) == oracle_py.ref_fir37(x)).all(), (n, kind)
+    import golden_vectors as gv
+    for key, x in gv.fir37_ref_inputs("cpu"):
+        assert gv.fir37_ref_output_equals(key, x, oracle_py.fir37_legacy(x, 0)), key
 
 def test_assembly_variant_is_the_plain_filter():
     """variant 1 (FIR37SSE_INLINE): y[n] = sat8((sum_k h[k] x[n + 8 - k]) >> 8) wherever the 16-bit lane tree does not saturate."""
@@ -51,7 +46,7 @@ def _chips_of_capture(name):
 def test_reference_sample_files_were_shaped_by_a_close_relative_of_this_filter(name):
     """kernel/HWTest/exe/tx samples/*.mf.bin: chips read off the file, through the restated filter -> within 3 LSB (1 Mbps; 4 LSB at 2 Mbps, whose chip
     levels the file does not let one read exactly) of the file everywhere, 60 % / 40 % of the samples exact.  (A least-squares fit of the taps from the file gives non-integer outer taps and a ripple longer than 37 taps, so the
-    files were not made by bbb_fir.c as it stands; this is evidence of kinship, not a pin.  The pin is oracle/_ref.)"""
+    files were not made by bbb_fir.c as it stands; this is evidence of kinship, not a pin.  The pin is the reference's compiled filter body.)"""
     y, chips = _chips_of_capture(name)
     out = oracle_py.fir37_legacy(chips, 0).astype(int)
     m = min(len(out), len(y)) - 64

@@ -2,10 +2,8 @@
 receive oracle cannot be pinned by one; instead the two halves of the reference's 802.11n code — modulator graphs and demodulator
 graph — are restated independently and played against each other here: every frame the transmit restatement makes must come out of
 the receive restatement bit for bit (L-SIG / HT-SIG fields, CRC-8, HT interleavers, stream parser, pilots, cyclic shifts)."""
-import os, re, zlib, numpy as np, pytest
+import zlib, numpy as np, pytest
 import oracle_py
-
-REF = "/root/reference"
 
 def _rx(o0, o1, chan=((1, 0), (0, 1)), noise=0.0, seed=0, lead=400, trail=300, cfo_hz=0.0):
     a = o0.astype(np.float64); b = o1.astype(np.float64)
@@ -66,17 +64,13 @@ def test_second_stream_is_a_cyclically_delayed_copy_in_the_legacy_part():
     assert (o0[h:h + 160] == -o0[h + 160:h + 320]).all() and (o1[h:h + 160] == o1[h + 160:h + 320]).all()
     assert (np.roll(o0[h + 32:h + 160], 16, axis=0) == o1[h + 32:h + 160]).all()
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_preamble_and_pilot_tables_vs_reference():
-    def table(path, name):
-        s = open(os.path.join(REF, "kernel/bb/Brick11/src", path)).read(); i = s.index(name + "[] ="); j = s.index("};", i)
-        return np.array(re.findall(r"\{\s*(-?\d+)\s*,\s*(-?\d+)\s*\}", s[i:j]), dtype=np.int16)
+    """The preamble tables of oracle/tx11n.cpp and the HT pilot polarity against the reference's _b_*.h tables (golden/ref_digests.json)."""
+    import golden_vectors as gv
     a, b, c, d = oracle_py.tx11n_preamble_tables()
-    assert (a == table("_b_lstf.h", "L_STF::_stf")).all() and (b == table("_b_lltf.h", "L_LTF::_ltf")).all()
-    assert (c == table("_b_htstf.h", "HT_STF::_stf")).all() and (d == table("_b_htltf.h", "HT_LTF::_ltf")).all()
+    assert gv.ref_table_equals("L_STF", a) and gv.ref_table_equals("L_LTF", b)
+    assert gv.ref_table_equals("HT_STF", c) and gv.ref_table_equals("HT_LTF", d)
     # the 127-entry pilot polarity table of the HT pilot generator is the 802.11a one (entry i = p(i+1)): x^7 + x^4 + 1 from all ones
-    s = open(os.path.join(REF, "kernel/bb/Brick11/src/_b_dot11_pilot.h")).read(); i = s.index("dot11_ofdm_pilot::_pilot_sign[pilot_size] ="); j = s.index("};", i)
-    sign = np.array([int(v) for v in re.findall(r"-?\d+", s[s.index("{", i):j])])
     st = 0x7F; seq = []
     for _ in range(127): o = ((st >> 6) ^ (st >> 3)) & 1; st = ((st << 1) | o) & 0x7F; seq.append(1 - 2 * o)
-    assert len(sign) == 127 and (sign == np.array([seq[(k + 1) % 127] for k in range(127)])).all()
+    assert gv.ref_table_equals("_pilot_sign", [seq[(k + 1) % 127] for k in range(127)])

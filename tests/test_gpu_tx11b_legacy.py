@@ -1,6 +1,6 @@
 """GPU parity tests for the legacy 802.11b transmit filter (pytest -m gpu): sb200_tx11b_fir37 and the BB11BPMDSpreadFIR4SSE / ...ASM entry
-points against oracle/tx11b_legacy.cpp, against the vectors the reference's own compiled code made (tests/golden/fir37) and, where
-oracle/_ref travelled with the snapshot, against that compiled code itself."""
+points against oracle/tx11b_legacy.cpp and against what the reference's own compiled code made: the vectors under tests/golden/fir37 and
+digests of its output on seeded inputs (tests/golden/ref_digests.json)."""
 import os, ctypes as C, numpy as np, pytest
 import oracle_py
 from sora_b200 import api
@@ -33,12 +33,10 @@ def test_device_matches_oracle_on_ragged_batches(eng, variant):
         assert (out[f, :n] == oracle_py.fir37_legacy(x[f, :n], variant)).all(), (f, n)
         assert (out[f, n:] == 99).all()                                                          # nothing outside a frame's own range is touched
 
-@pytest.mark.skipif(not oracle_py.ref_fir37_available(), reason="oracle/_ref was not built in the container this snapshot came from")
 def test_device_equals_the_compiled_reference_body(eng):
-    rng = np.random.default_rng(9)
-    for n in (8, 64, 4096, 100000 // 8 * 8):
-        x = rng.integers(-128, 128, (n, 2)).astype(np.int8)
-        assert (eng.tx11b_fir37(x, 0) == oracle_py.ref_fir37(x)).all(), n
+    import golden_vectors as gv
+    for key, x in gv.fir37_ref_inputs("gpu"):
+        assert gv.fir37_ref_output_equals(key, x, eng.tx11b_fir37(x, 0)), key
 
 def test_legacy_entry_points_and_errors(eng):
     lib = api.load_library()

@@ -3,7 +3,8 @@
 compare it with the closed-form generators used by oracle/ and sora_b200/csrc.
 
 Used two ways:
-  * tests/test_tables_vs_reference.py imports the parse_* helpers (skipped when /root/reference is absent)
+  * tests/golden/make_ref_digests.py digests the parsed tables into tests/golden/ref_digests.json, which the suite compares the
+    closed-form generators below with
   * `python tools/refcheck.py --emit-demap` regenerates sora_b200/csrc/demap_lut.inc (the only
     tables with no closed form: Brick11/src/demapper.h:56-130)
 """
